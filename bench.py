@@ -5,6 +5,7 @@
     python bench.py --config cfg2|cfg3|cfg4|cfg5                     # the other BASELINE.json configs (see CONFIGS)
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...      # one rank per GPU
     python bench.py --impl reference ...                             # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR                           # also write what the last timed step computed, DIR/<name>.npy
 
 torch.distributed.run is only the LAUNCHER: the rank processes never import torch.  The library builds its own NCCL communicator
 from RANK / WORLD_SIZE / LOCAL_RANK / MASTER_PORT (clip_b200_dist_init: ncclCommInitRank, unique id through a rendezvous file), and
@@ -141,6 +142,22 @@ class ClockSampler:
                 "power_w_max": max(pw) if pw else None, "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> what the last timed step handed its caller.  Written as float32 / float64 .npy, at most DUMP_BYTES in all: a larger
+    array is cut to a fixed, seeded sample of its rows (the same rows for the same arguments, so two builds compare row for row)."""
+    os.makedirs(path, exist_ok=True)
+    budget = DUMP_BYTES // len(arrays)
+    for name, a in arrays.items():
+        a = np.asarray(a, np.float32 if a.dtype == np.float32 else np.float64)
+        if a.nbytes > budget:
+            keep = budget // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def peaks():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -204,7 +221,7 @@ def run_reference_arm(args, cfg, rank):
     vals, base = [], None
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        base, _ = cpu_reference_sample(cfg, model, per_step, threads)
+        base, emb = cpu_reference_sample(cfg, model, per_step, threads)
         vals.append(base["value"])
     wall = time.perf_counter() - t0
     v = float(np.mean(vals))
@@ -219,6 +236,8 @@ def run_reference_arm(args, cfg, rank):
            "cpu_baseline": base, "e2e": {"value": v, "unit": unit, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
            "wall_s": wall}
     print(json.dumps(out), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {("text" if cfg["kind"] == "text" else "image") + "_embeddings": emb})
 
 
 # ---- GPU side -----------------------------------------------------------------------------------------------------------
@@ -255,6 +274,12 @@ class Bench:
         v = (C.c_double * 2)(ms_dev, ms_wall)
         assert L.clip_b200_dist_max_f64(ctx, v, 2)                  # max over ranks
         return v[0] / steps, v[1] / steps
+
+    def fetch(self, d_ptr, shape):
+        """float32 device buffer -> host array (after timed(), which synchronises)"""
+        a = np.empty(shape, np.float32)
+        assert self.L.clip_b200_memcpy_d2h(self.ctx, a.ctypes.data, d_ptr, a.nbytes), self.lib.last_error()
+        return a
 
     def drop_profile(self):
         for k in range(4):
@@ -306,11 +331,12 @@ def bench_image(b, units):
     launches = (L.clip_b200_kernel_launches(ctx) - l0) + (args.steps if world > 1 else 0)
     clocks = sampler.stop() if rank == 0 else None
     kinds = b.kinds(args.steps)
+    outputs = {"image_embeddings": b.fetch(d_all, (B * world, d))} if args.dump_outputs else None
     for _ in range(2):
         step_e2e()
     ms_e2e, _ = b.timed(step_e2e, max(2, args.steps // 2))
     b.drop_profile()
-    res = {"ms_step": ms_step, "ms_wall": ms_wall, "launches": launches, "clocks": clocks, "kinds": kinds,
+    res = {"outputs": outputs, "ms_step": ms_step, "ms_wall": ms_wall, "launches": launches, "clocks": clocks, "kinds": kinds,
            "e2e": {"value": B * world / (ms_e2e / 1e3), "unit": "img/s", "h2d_bytes_per_step": B * per * 4, "d2h_bytes_per_step": B * world * d * 4,
                    "ms_per_step": ms_e2e, "call": "clip_b200_image_batch_encode_all" if world > 1 else "clip_image_batch_encode",
                    "host_buffers": "pinned (cudaMallocHost)"}}
@@ -385,12 +411,13 @@ def bench_text(b, units):
     launches = (L.clip_b200_kernel_launches(ctx) - l0) + (args.steps if world > 1 else 0)
     clocks = sampler.stop() if rank == 0 else None
     kinds = b.kinds(args.steps)
+    outputs = {"text_embeddings": b.fetch(d_all, (TB * world, d))} if args.dump_outputs else None
     for _ in range(2):
         step_e2e()
     ms_e2e, _ = b.timed(step_e2e, max(2, args.steps // 2))
     b.drop_profile()
     T_pad = (TL + 7) // 8 * 8 if TL < 77 else 77
-    return {"ms_step": ms_step, "ms_wall": ms_wall, "launches": launches, "clocks": clocks, "kinds": kinds,
+    return {"outputs": outputs, "ms_step": ms_step, "ms_wall": ms_wall, "launches": launches, "clocks": clocks, "kinds": kinds,
             "e2e": {"value": TB * world / (ms_e2e / 1e3), "unit": "seq/s", "h2d_bytes_per_step": TB * T_pad * 4 + TB * 4,
                     "d2h_bytes_per_step": TB * world * d * 4, "ms_per_step": ms_e2e,
                     "call": "clip_b200_text_batch_encode_all" if world > 1 else "clip_text_batch_encode", "host_buffers": "pageable clip_tokens arrays"}}
@@ -438,12 +465,16 @@ def bench_zsl(b, n_img_global, n_lab_global):
     launches = (L.clip_b200_kernel_launches(ctx) - l0) + (args.steps if world > 1 else 0)
     clocks = sampler.stop() if rank == 0 else None
     kinds = b.kinds(args.steps)
+    outputs = None
+    if args.dump_outputs:       # this rank's images; the label embeddings are all ranks' (all-gathered)
+        outputs = {"image_embeddings": b.fetch(d_img, (B, d)), "label_embeddings": b.fetch(d_txt, (NL * world, d)),
+                   "top5_scores": scores.copy(), "top5_labels": idx.astype(np.float64)}
     for _ in range(2):
         step_e2e()
     same = bool(np.array_equal(idx, ref_idx))
     ms_e2e, _ = b.timed(step_e2e, max(2, args.steps // 2))
     b.drop_profile()
-    return {"ms_step": ms_step, "ms_wall": ms_wall, "launches": launches, "clocks": clocks, "kinds": kinds, "units": B,
+    return {"outputs": outputs, "ms_step": ms_step, "ms_wall": ms_wall, "launches": launches, "clocks": clocks, "kinds": kinds, "units": B,
             "e2e": {"value": B * world / (ms_e2e / 1e3), "unit": "img/s", "h2d_bytes_per_step": B * per * 4 + NL * 80 * 4,
                     "d2h_bytes_per_step": B * K * 8, "ms_per_step": ms_e2e, "call": "clip_b200_zero_shot_images",
                     "top5_identical_to_device_resident_path": same}}
@@ -486,6 +517,7 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--quick", action="store_true", help=argparse.SUPPRESS)        # skip the secondary legs (ncu captures, probes)
     ap.add_argument("--no-text", action="store_true", help=argparse.SUPPRESS)       # kept for old command lines: same as --quick
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy (rank 0; float32/float64, <= 64 MB)")
     args = ap.parse_args()
     args.quick = args.quick or args.no_text
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
@@ -553,6 +585,8 @@ def main():
             if k in res:
                 out[k] = res[k]
         print(json.dumps(out), flush=True)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, res["outputs"])
     b.sync_all()
     b.lib.free(b.ctx)
 

@@ -24,6 +24,12 @@ def golden(geom):
     return {k: z[k] for k in z.files}
 
 
+def reference_runs():
+    """What the reference returned for the inputs of the embedding and scoring tests (tests/golden/make_ref_golden.py)."""
+    z = np.load(os.path.join(GOLDEN, "reference_runs.npz"))
+    return {k: z[k] for k in z.files}
+
+
 def model_file(geom: str, ftype: str, prod: "bd.ClipLib") -> str:
     """(geom, SEED, ftype) -> path; f16/f32 written from the seed, q* made with the PRODUCT's clip_model_quantize
     (byte-identical to the reference's: tests/test_host_side.py)."""

@@ -1,6 +1,5 @@
-"""Host-side members of the interface (no GPU): file quantizer, weight re-tiling, tokenizer, preprocess -- each
-checked bit-exactly against vectors produced by the reference (tests/golden, oracle/_ref) and, when the reference
-library is present, against it live."""
+"""Host-side members of the interface (no GPU): file quantizer, weight re-tiling, tokenizer, preprocess, image decoders -- each
+checked bit-exactly against what the reference returned for the same inputs (tests/golden, recorded from oracle/_ref)."""
 import ctypes as C
 import hashlib
 import json
@@ -10,11 +9,44 @@ import numpy as np
 import pytest
 
 import binding as bd
-import ref_run
 import synth_gguf as sg
 from _util import FTYPES, GOLDEN, check_sha, golden, model_file
 
 HOST = json.load(open(os.path.join(GOLDEN, "host_ops.json")))
+
+
+def _sha(data):
+    return hashlib.sha256(data).hexdigest()
+
+
+def _reference_runs():
+    """What the reference returned for this module's inputs beyond host_ops.json and jpeg/ (tests/golden/make_ref_golden.py)."""
+    with open(os.path.join(GOLDEN, "reference_runs.json")) as f:
+        return json.load(f)
+
+
+class _ReferenceDecodes:
+    """What the reference's clip_image_load_from_file returned for each file a decoder test writes, in the order the test writes them
+    (sha256 of the pixels; of the file too where the encoder is lossy).  tests/golden/make_ref_golden.py records them by running the
+    same test with the reference library in place of this class."""
+
+    def __init__(self, test, pin_files=False):
+        self.test, self.want, self.n, self.pin_files = test, _reference_runs()["decodes"][test], 0, pin_files
+
+    def check(self, path, got):
+        assert self.n < len(self.want), (self.test, "more files than the recording")
+        file_sha, pix_sha = self.want[self.n]
+        if self.pin_files:
+            assert _sha(open(path, "rb").read()) == file_sha, (self.test, self.n, "the encoder wrote other bytes than when recorded")
+        assert got is not None and _sha(got.tobytes()) == pix_sha, (self.test, self.n)
+        self.n += 1
+
+    def done(self):
+        assert self.n == len(self.want), (self.test, self.n, len(self.want))
+
+
+def _reference_decodes(test, pin_files=False):
+    return _ReferenceDecodes(test, pin_files)
 
 
 @pytest.mark.parametrize("ft", ["q4_0", "q4_1", "q5_0", "q5_1", "q8_0"])
@@ -86,21 +118,18 @@ def test_preprocess_matches_reference_golden_bit_exactly(prod):
         assert hashlib.sha256(out.tobytes()).hexdigest() == e["sha256"], e
 
 
-@pytest.mark.skipif(not ref_run.available(), reason="oracle/_ref not built")
+LIVE_TEXTS = ["the red apple isn't a dog", "  double  spaces and 42 numbers!!", "mixed'case I'LL"]
+LIVE_IMAGE = (123, 77, 99)      # nx, ny, seed of _synth_u8
+
+
 def test_tokenizer_and_preprocess_match_live_reference(prod):
-    import subprocess, sys, tempfile
+    """Texts and an image outside host_ops.json, against the reference's tokens and preprocessed floats (tests/golden/reference_runs.json)."""
+    want = _reference_runs()["tokenize_preprocess"]
     model = model_file("tiny", "f16", prod)
-    texts = ["the red apple isn't a dog", "  double  spaces and 42 numbers!!", "mixed'case I'LL"]
-    u8 = _synth_u8(123, 77, 99)
-    code = ("import sys, json, numpy as np; sys.path.insert(0, %r); sys.path.insert(0, %r); import binding as bd, ref_run; r = bd.ClipLib(ref_run.REF_LIB); c = r.load(%r, 0);"
-            "print(json.dumps({'tok': [[int(v) for v in r.tokenize(c, t)] for t in %r], 'pre': r.preprocess(c, np.load(sys.argv[1])).ravel().tolist()}))"
-            % (os.path.join(os.path.dirname(GOLDEN), "..", "clip.cpp_b200"), os.path.join(os.path.dirname(GOLDEN), "..", "oracle"), model, texts))
-    with tempfile.NamedTemporaryFile(suffix=".npy") as f:
-        np.save(f.name, u8)
-        res = json.loads(subprocess.run([sys.executable, "-c", code, f.name], capture_output=True, text=True, check=True).stdout.strip().splitlines()[-1])
-    for t, ids in zip(texts, res["tok"]):
+    check_sha(model, want["model_sha"])
+    for t, ids in zip(LIVE_TEXTS, want["tokens"], strict=True):
         assert _tokenize(prod, model, t) == ids
-    assert np.array_equal(_preprocess(prod, u8).ravel(), np.array(res["pre"], np.float32))
+    assert _sha(_preprocess(prod, _synth_u8(*LIVE_IMAGE)).tobytes()) == want["preprocess_sha256"]
 
 
 def test_scoring_helpers_match_reference_arithmetic(prod):
@@ -151,19 +180,18 @@ def test_png_decode_matches_pil_and_rejects_unknown_formats(prod, tmp_path):
     assert _load_file(prod, g) is None and b"supported formats" in prod.lib.clip_b200_last_error()
 
 
-@pytest.mark.skipif(not ref_run.available(), reason="oracle/_ref not built")
 def test_png_decode_matches_live_reference(prod, tmp_path):
     Image = pytest.importorskip("PIL.Image")
     rng = np.random.default_rng(1)
-    ref = bd.ClipLib(ref_run.REF_LIB)
+    ref = _reference_decodes("png_pil")
     ims = {"g16.png": Image.fromarray(rng.integers(0, 65536, (11, 13), dtype=np.uint16)),
            "la.png": Image.fromarray(rng.integers(0, 256, (20, 31, 2), dtype=np.uint8), "LA"),
            "rgb.png": Image.fromarray(rng.integers(0, 256, (64, 48, 3), dtype=np.uint8))}
     for name, im in ims.items():
         p = str(tmp_path / name)
         im.save(p)
-        a, b = _load_file(prod, p), _load_file(ref, p)
-        assert a is not None and b is not None and np.array_equal(a, b), name
+        ref.check(p, _load_file(prod, p))
+    ref.done()
 
 
 def _write_png(path, arr, ctype, depth, interlace=False, palette=None):
@@ -255,9 +283,9 @@ def _png_expected(arr, ctype, depth, palette=None):
 
 def test_png_every_colour_type_depth_and_interlace(prod, tmp_path):
     """clip_image_load_from_file on PNGs PIL cannot write: packed 1/2/4-bit grey and palette, 16-bit, Adam7 -- against the pixel rule of
-    stb_image (computed here) and, when oracle/_ref is built, against the reference library itself."""
+    stb_image (computed here) and against what the reference library returned for each file."""
     rng = np.random.default_rng(11)
-    ref = bd.ClipLib(ref_run.REF_LIB) if ref_run.available() else None
+    ref = _reference_decodes("png_modes")
     pal = rng.integers(0, 256, (256, 3), dtype=np.uint8)
     n = 0
     for (w, h) in [(1, 1), (3, 2), (7, 9), (8, 8), (13, 5), (33, 17)]:
@@ -273,10 +301,10 @@ def test_png_every_colour_type_depth_and_interlace(prod, tmp_path):
                 got = _load_file(prod, p)
                 assert got is not None, (w, h, ctype, depth, interlace, prod.last_error())
                 assert np.array_equal(got, _png_expected(arr, ctype, depth, pal)), (w, h, ctype, depth, interlace)
-                if ref is not None:
-                    assert np.array_equal(got, _load_file(ref, p)), (w, h, ctype, depth, interlace)
+                ref.check(p, got)
                 n += 1
     assert n == 6 * 2 * 15
+    ref.done()
 
 
 def _bmp(w, h, bpp, row_fn, hsz=40, comp=0, masks=None, palette=None, topdown=False):
@@ -310,9 +338,9 @@ def _field(v, mask):
 
 def test_bmp_and_pnm_variants(prod, tmp_path):
     """clip_image_load_from_file on BMP (palettes of 1/4/8 bits, 16-bit 555 / 565 / 444, 24-bit, 32-bit, V3/V4/V5 and OS/2 headers,
-    top-down rows) and binary PGM / PPM: against the rule computed here and, when oracle/_ref is built, the reference library."""
+    top-down rows) and binary PGM / PPM: against the rule computed here and what the reference library returned for each file."""
     rng = np.random.default_rng(21)
-    ref = bd.ClipLib(ref_run.REF_LIB) if ref_run.available() else None
+    ref = _reference_decodes("bmp_pnm")
     p = str(tmp_path / "t.bin")
 
     def check(data, want, vs_ref=True):
@@ -320,8 +348,8 @@ def test_bmp_and_pnm_variants(prod, tmp_path):
         got = _load_file(prod, p)
         assert got is not None, prod.last_error()
         assert np.array_equal(got, want)
-        if ref is not None and vs_ref:
-            assert np.array_equal(got, _load_file(ref, p))
+        if vs_ref:
+            ref.check(p, got)
 
     for (w, h) in [(1, 1), (5, 3), (13, 7), (33, 10)]:
         for topdown in (False, True):
@@ -355,6 +383,7 @@ def test_bmp_and_pnm_variants(prod, tmp_path):
     rle[30] = 1                                                    # BI_RLE8: refused, as in the reference
     open(p, "wb").write(bytes(rle))
     assert _load_file(prod, p) is None
+    ref.done()
 
 
 def _gif_lzw(indices, min_bits, grow=True):
@@ -432,9 +461,9 @@ def _gif(W, H, gpal, frame, x0=0, y0=0, bg=0, transparent=None, interlace=False,
 def test_gif_first_frame(prod, tmp_path):
     """clip_image_load_from_file on GIF: the first frame as stb_image composes it (transparent pixels black, uncovered canvas = background
     colour when its index is non-zero -- with red and blue swapped, a quirk of the reference that is kept), interlaced rows, local
-    colour tables, both LZW styles; against the rule computed here and, when oracle/_ref is built, the reference library."""
+    colour tables, both LZW styles; against the rule computed here and what the reference library returned for each file."""
     rng = np.random.default_rng(31)
-    ref = bd.ClipLib(ref_run.REF_LIB) if ref_run.available() else None
+    ref = _reference_decodes("gif")
     p = str(tmp_path / "t.gif")
 
     def check(data, want):
@@ -442,8 +471,7 @@ def test_gif_first_frame(prod, tmp_path):
         got = _load_file(prod, p)
         assert got is not None, prod.last_error()
         assert np.array_equal(got, want)
-        if ref is not None:
-            assert np.array_equal(got, _load_file(ref, p))
+        ref.check(p, got)
 
     for (W, H) in [(1, 1), (7, 5), (33, 21), (120, 90)]:
         for ncol in (2, 16, 200, 256):
@@ -469,6 +497,7 @@ def test_gif_first_frame(prod, tmp_path):
                     check(_gif(W, H, pal, sub, x0=2, y0=1, bg=bg, interlace=True), want)
     open(p, "wb").write(b"GIF89a" + bytes(7) + b"\x3B")
     assert _load_file(prod, p) is None
+    ref.done()
 
 
 JPEG_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "jpeg")
@@ -489,13 +518,12 @@ def test_jpeg_decode_matches_reference_golden(prod):
         assert hashlib.sha256(got.tobytes()).hexdigest() == want["sha256"], (name, float(got.mean()), want["mean"])
 
 
-@pytest.mark.skipif(not ref_run.available(), reason="oracle/_ref not built")
 def test_jpeg_decode_matches_live_reference(prod, tmp_path):
-    """Same comparison against the reference library itself on freshly written files (sizes x sampling x mode x quality), and on the
-    two sample JPEGs the reference ships when its tree is present."""
+    """Same comparison on files PIL writes here (sizes x sampling x mode x quality), against what the reference library returned for
+    them, and on the two sample JPEGs the reference ships (tests/golden/jpeg/ref_*.jpg)."""
     Image = pytest.importorskip("PIL.Image")
     rng = np.random.default_rng(5)
-    ref = bd.ClipLib(ref_run.REF_LIB)
+    ref = _reference_decodes("jpeg_pil", pin_files=True)
     p = str(tmp_path / "t.jpg")
     n = 0
     for (w, h) in [(1, 1), (8, 8), (15, 9), (33, 17), (100, 75), (224, 224), (1234, 901)]:       # the last one is > 1 MP: threaded IDCT / colour rows
@@ -507,13 +535,12 @@ def test_jpeg_decode_matches_live_reference(prod, tmp_path):
                 for prog in (False, True):
                     q = int(rng.integers(5, 100))
                     Image.fromarray(pic).save(p, quality=q, subsampling=sub, progressive=prog, optimize=bool(n & 1))
-                    a, b = _load_file(prod, p), _load_file(ref, p)
-                    assert a is not None and b is not None and np.array_equal(a, b), (w, h, sub, prog, q)
+                    ref.check(p, _load_file(prod, p))
                     n += 1
-    for f in ("/root/reference/tests/red_apple.jpg", "/root/reference/tests/white.jpg"):
-        if os.path.exists(f):
-            a, b = _load_file(prod, f), _load_file(ref, f)
-            assert a is not None and np.array_equal(a, b), f
+    for name in ("ref_red_apple", "ref_white"):
+        f = os.path.join(JPEG_GOLDEN, name + ".jpg")
+        ref.check(f, _load_file(prod, f))
+    ref.done()
 
 
 def test_jpeg_decoder_survives_corrupt_files(prod, tmp_path):

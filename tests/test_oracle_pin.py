@@ -1,6 +1,6 @@
 """Pins the CPU oracle (oracle/clip_oracle.c + oracle.py) before it is trusted as the checker:
   1. against golden embeddings the REFERENCE produced (tests/golden/*.npz, made by oracle/_ref);
-  2. against the reference itself, live, when oracle/_ref/libclip_ref.so is present (build container + GPU box);
+  2. against the reference's embeddings of inputs outside those fixtures, un-normalised (tests/golden/reference_runs.npz);
   3. its block quantizer against the reference's quantized model files (sha256 of the whole GGUF).
 Tolerances: the oracle reproduces every rounding point of the reference, so only summation order differs; quantized
 paths re-quantize activations per layer, which turns ulp-level differences into occasional +-1 flips (observed 1e-5)."""
@@ -10,9 +10,8 @@ import numpy as np
 import pytest
 
 import oracle as orc
-import ref_run
 import synth_gguf as sg
-from _util import FTYPES, check_sha, golden, model_file, one_minus_cos, token_seqs
+from _util import FTYPES, check_sha, golden, model_file, one_minus_cos, reference_runs, token_seqs
 
 PIN_TOL = {"f32": 1e-5, "f16": 1e-5, "q4_0": 5e-4, "q4_1": 5e-4, "q5_0": 5e-4, "q5_1": 5e-4, "q8_0": 5e-4}
 
@@ -43,14 +42,22 @@ def test_oracle_matches_reference_golden_variants(prod, geom, ft):
     assert one_minus_cos(m.encode_text(seq), g["txt_" + ft][0]) <= PIN_TOL[ft]
 
 
-@pytest.mark.skipif(not ref_run.available(), reason="oracle/_ref not built (needs /root/reference at build time)")
-@pytest.mark.parametrize("ft", ["f16", "q4_1", "q5_0"])
+LIVE_FTYPES = ["f16", "q4_1", "q5_0"]
+
+
+def live_inputs():
+    """Inputs of test_oracle_matches_live_reference: seeds none of the golden fixtures above use."""
+    return sg.synth_images(2, 64, 31337), [sg.synth_tokens(1, n, 7 * n)[0] for n in (4, 50)]
+
+
+@pytest.mark.parametrize("ft", LIVE_FTYPES)
 def test_oracle_matches_live_reference(prod, ft):
-    """Fresh inputs (not in any fixture), reference run in its own process (see oracle/ref_run.py)."""
+    """Un-normalised embeddings of fresh inputs against the reference's (recorded by tests/golden/make_ref_golden.py)."""
     path = model_file("tiny", ft, prod)
-    imgs = sg.synth_images(2, 64, 31337)
-    seqs = [sg.synth_tokens(1, n, 7 * n)[0] for n in (4, 50)]
-    r = ref_run.run_reference(path, imgs, seqs, n_threads=2, normalize=False)
+    check_sha(path, golden("tiny")["sha_" + ft])
+    imgs, seqs = live_inputs()
+    g = reference_runs()
+    r = {"img": g["pin_img_" + ft], "txt": g["pin_txt_" + ft]}
     m = orc.OracleModel(path)
     for i in range(2):
         oi, ot = m.encode_image(imgs[i], normalize=False), m.encode_text(seqs[i], normalize=False)
